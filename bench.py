@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W                      # this implementation
     python bench.py --impl reference --gpus N --steps K --warmup W     # the reference's CPU read path (oracle port)
     python bench.py --config c4 --gpus N                               # model distribution: every GPU ends up with the whole file
+    python bench.py --gpus N --steps K --warmup W --dump-outputs DIR   # also write the last step's outputs to DIR/*.npy (seeded inputs)
     (N > 1: launched by torchrun, one rank per GPU)
 
 Workload (config C2 of BASELINE.json per GPU, scaled weakly: C3's shape at N=8): synthetic files of N x 16 GiB in 4 MiB
@@ -74,7 +75,12 @@ def parse():
     ap.add_argument("--dir", default="")
     ap.add_argument("--no-memory-guard", action="store_true", help="do not shrink --gib-per-gpu when the stores would not fit into the container's memory")
     ap.add_argument("--ref-materialize-gib", type=float, default=64.0, help="reference arm: how much of the file's head is written to the store (the CPU reader never reads past its sample)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default="", metavar="DIR", help="after the timed steps, write what the last headline step returned as DIR/<name>.npy (see dump_outputs); "
+                                                                     "refused when the memory guard would shrink --gib-per-gpu, so the same arguments always read the same files")
+    args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.config != "c2"):
+        ap.error("--dump-outputs applies to the headline read (--impl ours --config c2)")
+    return args
 
 
 class ClockSampler:
@@ -327,6 +333,35 @@ def timed_read(fs, path, rank, world, dst, shard_bytes, stream):
     return a.elapsed_time(b), a2.elapsed_time(b2), s, stats
 
 
+DUMP_SAMPLE = 4 << 20  # bytes of HBM output --dump-outputs keeps, over all ranks (16 MiB as float32)
+
+
+def dump_positions(shard_bytes, world):
+    """Offsets into a rank's shard that --dump-outputs samples: seeded, sorted, the same for every run and build at this size."""
+    import numpy as np
+    return np.sort(np.random.default_rng(0).integers(0, shard_bytes, min(shard_bytes, DUMP_SAMPLE // world)))
+
+
+def dump_outputs(out_dir, rank, world, dst, sum_crc):
+    """What a caller of the timed path holds after the last headline step, as .npy files two builds can be compared by:
+         bytes_sample     float32  the HBM bytes at dump_positions()
+         block_byte_sums  float64  the sum of the bytes of every 4 MiB block of the shard (every byte counts, exact in float64)
+         crc_sum          float64  the sum of the per-block CRCs cv_verify returned (its mismatch count was asserted to be 0)
+    Several ranks: one set per rank, names suffixed _rank<r>."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    pos = torch.from_numpy(dump_positions(dst.numel(), world)).to(dst.device)
+    chunk = 64 * BLOCK  # the reduction may widen its input first: 256 MiB at a time; a block sums to < 2**31
+    sums = torch.cat([dst[i:i + chunk].view(-1, BLOCK).sum(dim=1, dtype=torch.int32) for i in range(0, dst.numel(), chunk)])
+    arrays = {"bytes_sample": dst[pos].cpu().numpy().astype(np.float32),
+              "block_byte_sums": sums.cpu().numpy().astype(np.float64),
+              "crc_sum": np.array([sum_crc], dtype=np.float64)}
+    suffix = "_rank%d" % rank if world > 1 else ""
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), a)
+
+
 def run_leg(name, cluster, fs, tier, args, rank, world, dist, dst, shard_bytes, steps, warmup, fresh, inode0, pool=None):
     """steps+warmup passes; fresh=True: every pass reads a file written just before it (never read by anyone), and the file of
     `pool` passes ago is dropped; fresh=False: one file, read again and again.  -> dict(e2e_ms[], ingest_ms[], warm_ms[], stats)."""
@@ -391,6 +426,8 @@ def main():
         args.gib_per_gpu = pick[0]
         if args.gib_per_gpu != asked_gib and rank == 0:
             log("memory guard: %g GiB per GPU does not fit into 70%% of %s; running %g GiB per GPU" % (asked_gib, budget_sources, args.gib_per_gpu))
+        if args.dump_outputs and args.gib_per_gpu != asked_gib:  # a dump of another size cannot be compared with one taken at the asked size
+            raise SystemExit("--dump-outputs: the memory guard cut --gib-per-gpu %g to %g; ask for a size this host holds" % (asked_gib, args.gib_per_gpu))
     shard_bytes = int(args.gib_per_gpu * (1 << 30)) // BLOCK * BLOCK
     n_total = shard_bytes * world
     my_blocks = shard_bytes // BLOCK
@@ -426,6 +463,8 @@ def main():
         head = run_leg("fresh", cluster, fs, args.tier, args, rank, world, dist, dst, shard_bytes, args.steps, args.warmup, True, 5000)
         launches = (K.launch_count() - launches0) * args.steps // max(1, args.steps + args.warmup)
         arena1 = fs.arena_stats()
+        if args.dump_outputs:  # before the side legs overwrite dst
+            dump_outputs(args.dump_outputs, rank, world, dst, head["sum_crc"])
         # ---- side legs
         legs = set(x for x in args.legs.split(",") if x) if side > 0 else set()
         if world > 1:  # beyond one GPU the side legs are the re-read and the kernel-only pass; the transport legs are one-GPU numbers

@@ -197,7 +197,11 @@ Err ClusterConf::from_string(const std::string& toml, ClusterConf* c) {
             else if (k == "register_when_idle") b.register_when_idle = as_bool(v);
             else if (k == "gds") {
                 const std::string m = unquote(v);
-                b.gds = (m == "on" || m == "true" || m == "1") ? 1 : (m == "off" || m == "false" || m == "0") ? 0 : 2;
+                if (m == "off" || m == "false" || m == "0") b.gds = false;
+                else if (m == "auto") b.gds = true;
+                else if (m == "on" || m == "true" || m == "1")
+                    e = Err::common("gds = \"" + m + "\" (cuFile's compatibility mode) is not supported: use \"auto\" (GPUDirect Storage where nvidia-fs is loaded) or \"off\"");
+                else e = Err::common("gds must be \"off\" or \"auto\": " + m);
             } else if (k == "local_unix_socket") b.local_unix_socket = as_bool(v);
             else if (k == "socket_buffer") e = as_size(v, &b.socket_buffer);
             else if (k == "arena") b.arena = as_bool(v);

@@ -64,9 +64,9 @@ struct B200Conf {
     int64_t arena_register_slice = 256ll << 20;  // one cudaHostRegister call covers this much of a segment (slices go to register_threads)
     bool local_unix_socket = false;  // block connections to a worker on this host use its abstract unix socket (net.h) instead of loopback TCP
     int64_t socket_buffer = 0;       // explicit SO_RCVBUF/SO_SNDBUF for block connections (0 = kernel autotuning)
-    int gds = 2;                  // "gds" = "off" | "on" | "auto": short-circuit reads of SSD/HDD/DISK-tier blocks go through cuFileRead
-                                  // (gds.h) straight into HBM; auto (default) = only with real GPUDirect Storage (nvidia-fs), on = also in
-                                  // cuFile's compatibility mode; anything GDS cannot serve goes through the pinned ring
+    bool gds = true;              // "gds" = "off" | "auto" (default): with auto, short-circuit reads of SSD/HDD/DISK-tier blocks go through
+                                  // cuFileRead (gds.h) straight into HBM where GPUDirect Storage (nvidia-fs) is loaded; anything GDS
+                                  // cannot serve goes through the pinned ring
     int numa_node = -1;           // bind fetch threads to this node's CPUs (-1: the GPU's node if discoverable, -2: no binding)
 };
 

@@ -53,6 +53,10 @@ std::unordered_map<std::string, Entry> g_files;
 
 std::string g_refusal;  // first reason a file was turned away (under g_mu)
 
+bool nvidia_fs_loaded() {
+    return access("/proc/driver/nvidia-fs/stats", R_OK) == 0;  // the nvidia-fs module publishes this file
+}
+
 void probe() {
     const char* names[] = {"libcufile.so.0", "libcufile.so", "/usr/local/cuda/lib64/libcufile.so.0", "/usr/local/cuda/lib64/libcufile.so"};
     for (const char* n : names)
@@ -75,13 +79,20 @@ void probe() {
         return;
     }
     g_info.available = true;
-    g_info.compat = access("/proc/driver/nvidia-fs/stats", R_OK) != 0;  // the nvidia-fs module publishes this file
-    g_info.detail = g_info.compat ? "cuFile compatibility mode (nvidia-fs kernel module not loaded)" : "GPUDirect Storage (nvidia-fs)";
+    g_info.detail = "GPUDirect Storage (nvidia-fs)";
 }
 
 }  // namespace
 
 const GdsInfo& gds_info() {
+    // Without nvidia-fs cuFile could only run in its compatibility mode, which is slower than the pinned ring; and opening cuFile's
+    // driver on a B200 without nvidia-fs stalled the first short-circuit read of a process for more than three minutes (observed in
+    // one test run).  The library is then not loaded at all.
+    static const bool native = nvidia_fs_loaded();
+    if (!native) {
+        static const GdsInfo closed{false, true, "nvidia-fs kernel module not loaded: cuFile is not opened, disk-tier blocks take the pinned ring"};
+        return closed;
+    }
     std::call_once(g_once, probe);
     return g_info;
 }
@@ -105,7 +116,8 @@ void gds_forget(const std::string& path) {
 }
 
 Err gds_read(const std::string& path, void* d_dst, int64_t n, int64_t file_off) {
-    if (!gds_info().available) return Err(kUnsupported, "GDS unavailable: " + g_info.detail);
+    const GdsInfo& gi = gds_info();
+    if (!gi.available) return Err(kUnsupported, "GDS unavailable: " + gi.detail);
     Entry e;
     {
         struct stat st;
@@ -120,9 +132,8 @@ Err gds_read(const std::string& path, void* d_dst, int64_t n, int64_t file_off) 
         }
         if (it == g_files.end()) {
             Entry ne;
-            // real GDS wants O_DIRECT; the compatibility mode does plain preads at whatever offset the caller asks for, which an
-            // O_DIRECT descriptor would refuse unless 512-byte aligned
-            ne.fd = g_info.compat ? -1 : ::open(path.c_str(), O_RDONLY | O_DIRECT | O_CLOEXEC);
+            // GDS wants O_DIRECT; a file system that refuses it gets a plain descriptor, and cuFileHandleRegister decides
+            ne.fd = ::open(path.c_str(), O_RDONLY | O_DIRECT | O_CLOEXEC);
             if (ne.fd < 0) ne.fd = ::open(path.c_str(), O_RDONLY | O_CLOEXEC);
             if (ne.fd < 0) return Err::io(str_printf("open %s: %s", path.c_str(), strerror(errno)));
             CvCuFileDescr d;

@@ -1117,7 +1117,7 @@ Err GpuFsReader::run_jobs(const std::vector<Job>& jobs, uint8_t* d_dst, void* us
         for (size_t j = g * k; j < std::min(J, g * k + k); j++) group_verbatim[g] |= mode[j] == kFramed;
     std::vector<int64_t> req_ids(J, 0);
     std::atomic<bool> use_mapped{bc.zero_copy};
-    std::atomic<bool> use_gds{!call_framed && bc.gds != 0 && gds_info().available && (bc.gds == 1 || !gds_info().compat)};
+    std::atomic<bool> use_gds{!call_framed && bc.gds && gds_info().available};
     std::atomic<uint64_t> gds_bytes{0};
     std::mutex held_mu;
     const int T_threads = static_cast<int>(std::min<size_t>(static_cast<size_t>(std::max(1, bc.fetch_threads)), NG));

@@ -26,7 +26,7 @@ def _check(rc: int):
 
 
 def gds_info() -> dict:
-    """GPUDirect Storage probe (gds.h): {available, compat, detail}."""
+    """GPUDirect Storage probe (gds.h): {available, compat (no nvidia-fs: cuFile not opened), detail}."""
     a = (ctypes.c_int64 * 2)()
     _check(_lib.lib().cv_gds_info(a))
     return {"available": bool(a[0]), "compat": bool(a[1]), "detail": _lib.lib().cv_last_error().decode(errors="replace")}

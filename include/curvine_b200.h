@@ -137,8 +137,9 @@ typedef struct CvReadStats {
     uint64_t reg_bytes;            /* bytes registered through the cache right now (<= register_cache) */
     uint64_t gds_bytes;            /* bytes read file -> HBM by cuFileRead (disk tiers, [b200] gds) */
 } CvReadStats;
-/* GPUDirect Storage probe: out[0] = 1 when libcufile loaded and its driver opened, out[1] = 1 when it runs in compatibility
- * mode (no nvidia-fs kernel module).  The message (cv_last_error) carries the detail either way. */
+/* GPUDirect Storage probe: out[0] = 1 when libcufile loaded and its driver opened, out[1] = 1 when the nvidia-fs kernel module is
+ * not loaded (cuFile would only have its compatibility mode, which is not used: libcufile is not loaded and out = {0, 1}).  The
+ * message (cv_last_error) carries the detail either way. */
 int64_t cv_gds_info(int64_t out[2]);
 int64_t cv_device_stats(cv_reader* r, CvReadStats* out);
 

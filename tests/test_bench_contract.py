@@ -76,6 +76,39 @@ def test_own_arm_control_flow_and_json_line_on_the_mock_runtime():
     assert c["kind"] == "port" and c["unit"] == "GB/s" and c["value"] > 0 and c["cores"] >= 2 and "pass" in c["sample"]
 
 
+def test_dump_outputs_are_the_last_steps_bytes_and_repeat_run_to_run(tmp_path):
+    """--dump-outputs DIR: after the timed steps the bench writes what the last headline step put into HBM (a seeded byte sample and
+    per-block byte sums) and the CRC sum cv_verify returned, as float .npy files.  Two runs with the same arguments write the same
+    arrays, and they are the oracle's bytes of the file the last timed step read."""
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
+    from oracle import clib, synth
+    env = _shim_env()
+    gib, steps, warmup, block = 1.0 / 16, 2, 1, 4 << 20
+    dumps = []
+    for k in range(2):
+        d = tmp_path / str(k)
+        p = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "mock_cuda", "run_bench_on_mock.py"), "--gib-per-gpu", str(gib), "--steps", str(steps),
+                            "--warmup", str(warmup), "--side-steps", "0", "--no-cpu-baseline", "--dump-outputs", str(d)],
+                           stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=900, env=env, cwd=ROOT)
+        assert p.returncode == 0, p.stderr[-3000:]
+        assert json.loads(p.stdout.strip().splitlines()[-1])["steps"] == steps
+        dumps.append({f: np.load(str(d / f)) for f in os.listdir(str(d))})
+    assert set(dumps[0]) == {"bytes_sample.npy", "block_byte_sums.npy", "crc_sum.npy"}
+    assert sum(a.nbytes for a in dumps[0].values()) <= 64 << 20
+    for name, a in dumps[0].items():
+        assert a.dtype in (np.float32, np.float64), name
+        np.testing.assert_array_equal(a, dumps[1][name], err_msg=name)
+    n = int(gib * (1 << 30))
+    want = np.frombuffer(synth.file_bytes(5000 + warmup + steps - 1, n, block), dtype=np.uint8)  # run_leg's inode of the last timed step
+    pos = bench.dump_positions(n, 1)
+    assert pos.size == bench.DUMP_SAMPLE
+    np.testing.assert_array_equal(dumps[0]["bytes_sample.npy"], want[pos].astype(np.float32))
+    np.testing.assert_array_equal(dumps[0]["block_byte_sums.npy"], want.reshape(-1, block).sum(axis=1, dtype=np.int64).astype(np.float64))
+    assert dumps[0]["crc_sum.npy"].tolist() == [float(clib.crc_blocks(1, want, block).astype(np.uint64).sum())]
+
+
 def test_own_arm_two_ranks_on_the_mock_runtime():
     """The N>1 launch the driver uses (torch.distributed.run, one rank per GPU) with world_size 2 on CPU: gloo stands in for NCCL, the
     mock runtime for the GPUs.  Rank 0 hosts the worker and generates the 2 x 0.25 GiB file, the manifest is broadcast, every rank

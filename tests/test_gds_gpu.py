@@ -1,5 +1,5 @@
-"""SSD-tier blocks into HBM: GPUDirect Storage (cuFileRead, curvine_b200/csrc/host/gds.h) where the box offers it -- also in
-cuFile's compatibility mode with gds = "on" -- and the pinned ring otherwise.  Whatever path runs, bytes and CRCs must equal the
+"""SSD-tier blocks into HBM: GPUDirect Storage (cuFileRead, curvine_b200/csrc/host/gds.h) where the box offers it (nvidia-fs loaded)
+and the pinned ring otherwise.  Whatever path runs, bytes and CRCs must equal the
 oracle's (SURVEY.md 8f-2; tier model: storage_info.rs:36-49, local_file.rs:202-213)."""
 import os
 import shutil
@@ -14,13 +14,9 @@ from oracle import clib, synth
 pytestmark = pytest.mark.gpu
 
 
-@pytest.mark.parametrize("gds", ["on", "off", "auto"])
+@pytest.mark.parametrize("gds", ["off", "auto"])
 def test_ssd_tier_file_lands_bit_exact_whichever_path_serves_it(cuda, gds):
     import torch
-    if gds == "on" and not os.environ.get("CV_TEST_GDS_ON") and not os.environ.get("CV_TEST_MOCK_CUDA_LIB"):
-        # cuFile's compatibility mode could not be exercised on a B200 box before round 2 lost its GPU access (the one attempt was
-        # refused at cuFileHandleRegister and fell back to the ring, as designed): forcing it stays opt-in until it has been seen to work
-        pytest.skip("gds = on (cuFile compatibility mode) is opt-in: CV_TEST_GDS_ON=1")
     d = tempfile.mkdtemp(prefix="cvssd", dir=os.environ.get("CV_SSD_DIR", "/tmp"))  # a disk-backed directory, not tmpfs
     try:
         with F.MiniWorker(["[SSD]" + d]) as w:
@@ -41,7 +37,7 @@ def test_ssd_tier_file_lands_bit_exact_whichever_path_serves_it(cuda, gds):
                 assert got == n - 12345 and bad == 0 and ver == 6  # block 0 is partial
                 assert dst[:got].cpu().numpy().tobytes() == want[12345:]
                 st = r.device_stats()
-                may_gds = info["available"] and (gds == "on" or (gds == "auto" and not info["compat"]))
+                may_gds = info["available"] and gds == "auto"
                 # either every byte went through cuFileRead, or cuFile turned the files away and every byte took the pinned ring
                 assert st["gds_bytes"] in ((0, got) if may_gds else (0,)), (st["gds_bytes"], F.gds_info(), gds)
                 r.complete()
@@ -53,6 +49,33 @@ def test_ssd_tier_file_lands_bit_exact_whichever_path_serves_it(cuda, gds):
                 assert got == n and bad == 0 and ver == 7
                 assert s == int(clib.crc_blocks(1, np.frombuffer(want, dtype=np.uint8), bs).astype(np.uint64).sum())
                 assert dst.cpu().numpy().tobytes() == want
+                r.complete()
+    finally:
+        shutil.rmtree(d, ignore_errors=True)
+
+
+def test_ssd_tier_file_lands_bit_exact_over_frames(cuda):
+    """short_circuit = false: the worker reads the SSD-tier block files and sends them as frames, which K2 unpacks and CRCs on the GPU.
+    cuFile never serves a framed read, whatever [b200] gds says."""
+    import torch
+    d = tempfile.mkdtemp(prefix="cvssdf", dir=os.environ.get("CV_SSD_DIR", "/tmp"))  # a disk-backed directory, not tmpfs
+    try:
+        with F.MiniWorker(["[SSD]" + d]) as w:
+            n, bs, ino = (24 << 20) + 4097, 4 << 20, 8802
+            man = w.create_file("/ssdf", ino, n, bs, storage_type=1)
+            want = synth.file_bytes(ino, n, bs)
+            conf = F.client_conf(short_circuit=False, b200='fetch_threads = 4\nverify_batch = 4\npinned_slots = 16\ncopy_group = 1\ngds = "auto"\n')
+            with F.CurvineFileSystem(conf) as fs:
+                fs.load_namespace(man)
+                dst = torch.full((n,), 0x11, dtype=torch.uint8, device=cuda)
+                r = fs.open("/ssdf")
+                got = r.read_device(dst.data_ptr(), n, torch.cuda.current_stream().cuda_stream)
+                s, bad, ver = r.verify()
+                torch.cuda.synchronize()
+                assert got == n and bad == 0 and ver == 7
+                assert s == int(clib.crc_blocks(1, np.frombuffer(want, dtype=np.uint8), bs).astype(np.uint64).sum())
+                assert dst.cpu().numpy().tobytes() == want
+                assert r.device_stats()["gds_bytes"] == 0
                 r.complete()
     finally:
         shutil.rmtree(d, ignore_errors=True)

@@ -823,3 +823,31 @@ def test_headers_are_plain_c_and_the_c_example_links_against_the_library_alone()
         open(os.path.join(d, "conf.toml"), "w").write(F.client_conf())
         e = subprocess.run([os.path.join(d, "c_host"), os.path.join(d, "conf.toml"), "/nope"], stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)
         assert e.returncode == 1 and "cv_open" in e.stdout, e.stdout
+
+def test_gds_probe_does_not_open_cufile_without_nvidia_fs(tmp_path):
+    """gds.h: without the nvidia-fs module cuFile is never read through, so the probe neither loads libcufile nor opens its driver (on a
+    B200 without nvidia-fs that stalled the first short-circuit read of a process for more than three minutes, observed in one test run):
+    {available: False, compat: True}, and no cufile.log appears in the working directory.  Run in a subprocess: the probe is once per process."""
+    if os.path.exists("/proc/driver/nvidia-fs/stats"):
+        pytest.skip("nvidia-fs is loaded: the probe opens cuFile here by design")
+    code = r'''
+import sys
+sys.path.insert(0, %r)
+from curvine_b200 import fs as F
+i = F.gds_info()
+print(i["available"], i["compat"], any("libcufile" in l for l in open("/proc/self/maps")))
+''' % os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    r = subprocess.run([sys.executable, "-c", code], stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True, timeout=120, cwd=str(tmp_path))
+    assert r.returncode == 0 and r.stdout.split()[-3:] == ["False", "True", "False"], r.stdout[-2000:]
+    assert not os.path.exists(str(tmp_path / "cufile.log"))
+
+
+@pytest.mark.parametrize("mode", ["on", "true", "sometimes"])
+def test_gds_accepts_only_off_and_auto(mode):
+    """[b200] gds: "off" and "auto" (the default) parse; "on" -- cuFile's compatibility mode, which is not used -- and anything else are refused
+    by name instead of being read as another mode."""
+    for ok in ("off", "auto"):
+        F.CurvineFileSystem(F.client_conf(b200='gds = "%s"\n' % ok)).close()
+    with pytest.raises(F.FsError) as e:
+        F.CurvineFileSystem(F.client_conf(b200='gds = "%s"\n' % mode))
+    assert "gds" in str(e.value) and mode in str(e.value), str(e.value)

@@ -20,7 +20,7 @@ MOCK = bool(os.environ.get("CV_TEST_MOCK_CUDA_LIB"))  # host-side stand-ins (tes
 def _need_two():
     import torch
     if not MOCK and torch.cuda.device_count() < 2:
-        pytest.skip("needs >= 2 CUDA devices (run with gpurun --gpus 2)")
+        pytest.skip("needs >= 2 CUDA devices")
     return torch
 
 

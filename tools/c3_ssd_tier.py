@@ -4,7 +4,7 @@
   warm   page cache holds the file (what a second pass over a recently written/read file sees)
 and the same two cases for the reference-shaped CPU reader (oracle/cpu_reader.c), host cores stated; beside them
   disk   the disk's own ceiling for this access pattern: the same block files read cold with O_DIRECT by 16 threads (a dd/fio stand-in)
-  gds    [b200] gds = on|off|auto: cuFileRead straight into HBM (curvine_b200/csrc/host/gds.h) vs the pinned ring
+  gds    [b200] gds = off|auto: cuFileRead straight into HBM (curvine_b200/csrc/host/gds.h) vs the pinned ring
   hbm    (--hbm) the worker's HBM tier over the SSD tier: framed reads cold from the disk, then -- after asynchronous promotion
          (hbm_promote_after = 1) -- served out of HBM as K4-packed frames; hit rate and GB/s per pass.
 BASELINE.json names 128 GiB over 8 GPUs; the GPU box has a 79 GB overlay disk, so the size is a parameter (default 16 GiB)."""

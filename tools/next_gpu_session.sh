@@ -29,8 +29,8 @@ run c5 400 python bench.py --config c5 --gpus 1
 run kbench_default 300 python tools/kbench.py --gib 4
 run kbench_copy_tile4 300 python tools/kbench.py --gib 4 --tile-copy 4
 run kbench_staged 300 python tools/kbench.py --gib 4 --staged 1
-# 4. SSD tier: GDS (direct if the box has nvidia-fs, else compat) against the pinned ring, and the HBM tier over it
-run c3_gds 600 python tools/c3_ssd_tier.py --gib 8 --gds on --hbm 2
+# 4. SSD tier: GDS (where the box has nvidia-fs; else the pinned ring) against the pinned ring, and the HBM tier over it
+run c3_gds 600 python tools/c3_ssd_tier.py --gib 8 --gds auto --hbm 2
 # 5. one ncu capture of the K2 walker and the launch list of a short bench (never a bench value)
 run ncu_launches 600 ncu --metrics gpu__time_duration.sum --clock-control none -c 400 --csv --log-file $O/next_launches.csv python bench.py --gpus 1 --steps 2 --warmup 1 --side-steps 0 --legs resident
 run ncu_k2 600 ncu --set full --clock-control none --import-source on -k regex:walk_kernel -c 4 -o $O/next_k2 python tools/kbench.py --gib 1 --only k2 --iters 2 --warm-sec 0
